@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- InternVLA-N1 policy-steps/sec on B200 (BASELINE.json metric), one JSON line on rank 0.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`, SURVEY.md §8d):
   dual_system    configs[3] (DEFAULT -- the configuration the metric is quoted on): the full dual-system step for 64
@@ -332,6 +332,25 @@ def _timing_tools(dev, world):
     return barrier, timed
 
 
+def _keep_last(fn, box):
+    """`fn` for a timed loop, keeping what its last call returned in box["out"] (--dump-outputs)."""
+    def step():
+        box["out"] = fn()
+    return step
+
+
+def dump_outputs(args, rank, name, out):
+    """--dump-outputs DIR: the output of the last timed step as DIR/<name>.npy in float32, on rank 0.  The inputs are
+    seeded, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    if not args.dump_outputs or rank != 0:
+        return
+    a = out.detach().float().cpu().numpy()
+    assert a.nbytes <= 64 << 20, (name, a.shape)
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+
+
 def run_ours_dual(args, wl):
     import torch.distributed as dist
     from internnav_b200 import _lib
@@ -368,12 +387,14 @@ def run_ours_dual(args, wl):
         step_resident()
     _lib.prof_read()
     barrier()
+    last = {}
     with ClockSampler(local) as clk:
-        ms = timed(step_resident, args.steps)
+        ms = timed(_keep_last(step_resident, last), args.steps)
     barrier()
     launches = _lib.prof_read()
     launches["total_launches"] //= max(args.steps, 1)
     clocks = clk.summary()
+    dump_outputs(args, rank, "trajectories", last["out"])
     step_e2e()
     barrier()
     ms_e2e = timed(step_e2e, args.steps, use_events=False)
@@ -478,12 +499,14 @@ def run_ours_s2(args, wl):
         step_resident()
     _lib.prof_read()
     barrier()
+    last = {}
     with ClockSampler(local) as clk:
-        ms = timed(step_resident, args.steps)
+        ms = timed(_keep_last(step_resident, last), args.steps)
     barrier()
     launches = _lib.prof_read()
     launches["total_launches"] //= max(args.steps, 1)
     clocks = clk.summary()
+    dump_outputs(args, rank, "latents", last["out"])
     step_e2e()
     barrier()
     ms_e2e = timed(step_e2e, args.steps, use_events=False)
@@ -583,12 +606,14 @@ def run_ours_train(args, wl):
     _lib.prof_read()
     exch.clear()
     barrier()
+    last = {}
     with ClockSampler(local) as clk:
-        ms = timed(step_resident, args.steps)
+        ms = timed(_keep_last(step_resident, last), args.steps)
     barrier()
     launches = _lib.prof_read()
     launches["total_launches"] //= max(args.steps, 1)
     clocks = clk.summary()
+    dump_outputs(args, rank, "loss", last["out"])
     exch_t = [e for e in exch if e]
     step_e2e()
     barrier()
@@ -712,11 +737,13 @@ def run_ours_denoise(args, wl):
         step_resident()
     _lib.prof_read()
     barrier()
+    last = {}
     with ClockSampler(local) as clk:
-        ms = timed(step_resident, args.steps)
+        ms = timed(_keep_last(step_resident, last), args.steps)
     barrier()
     launches = _lib.prof_read()
     clocks = clk.summary()
+    dump_outputs(args, rank, "trajectories", last["out"])
     for _ in range(2):
         step_e2e()
     barrier()
@@ -813,11 +840,13 @@ def run_ours_nextdit(args, wl):
         step_resident()
     _lib.prof_read()
     barrier()
+    last = {}
     with ClockSampler(local) as clk:
-        ms = timed(step_resident, args.steps)
+        ms = timed(_keep_last(step_resident, last), args.steps)
     barrier()
     launches = _lib.prof_read()
     clocks = clk.summary()
+    dump_outputs(args, rank, "trajectories", last["out"])
     for _ in range(2):
         step_e2e()
     barrier()
@@ -1027,7 +1056,7 @@ def eager_gpu_measure(wl, batch, steps, warmup, dev=None):
 def run_eager_gpu(args, wl):
     """--impl eager [--batch B]: the same-GPU PyTorch-eager baseline (default B = the workload's batch, 64)."""
     B = args.batch or wl["B"]
-    r = eager_gpu_measure(wl, B, max(args.steps, 2), max(args.warmup, 1))
+    r = eager_gpu_measure(wl, B, args.steps, max(args.warmup, 1))
     out = {"metric": "InternVLA-N1 policy-steps/sec (batch RGB-D+text->action)", "value": r["value"], "unit": "policy-steps/s",
            "impl": "eager_gpu", "n_gpus": 1, "steps": r["steps"], "warmup": max(args.warmup, 1), "ms_per_step": r["ms_per_step"],
            "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "bf16", "data": "synthetic",
@@ -1063,7 +1092,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true", help="skip the same-GPU PyTorch-eager baseline leg (N = 1)")
     ap.add_argument("--batch", type=int, default=0, help="--impl eager: environments per call (default: the workload's)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the output of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the output of --impl ours")
     _claim_stdout()
     wl = WORKLOADS[args.workload]
     if args.impl == "eager":

@@ -1,11 +1,23 @@
 """Host-side behaviour of the mirror classes that needs no GPU: argument handling, padding rules, error paths."""
 import ctypes
+import os
+import subprocess
+import sys
 from types import SimpleNamespace
 
 import pytest
 import torch
 
 from internnav_b200.internvla_n1 import IMAGE_TOKEN_INDEX, TRAJ_TOKEN_INDEX, InternVLAN1ForCausalLM
+
+
+def _rerun_without_gpu(name):
+    """Runs test `name` of this file in a child pytest that sees no CUDA device, so the no-device path is also checked on a
+    machine that has one."""
+    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", "%s::%s" % (__file__, name)],
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), cwd=os.path.dirname(__file__), capture_output=True,
+                       text=True)
+    assert r.returncode == 0 and " passed" in r.stdout, r.stdout + r.stderr
 
 
 class FakeS2:
@@ -78,7 +90,8 @@ def test_resize_plan_needs_a_device():
     from internnav_b200 import _lib
     from internnav_b200.preprocess import FramePreprocessor, _bind
     if torch.cuda.is_available():
-        pytest.skip("GPU present")
+        _rerun_without_gpu("test_resize_plan_needs_a_device")
+        return
     L = _lib.lib()
     _bind(L)
     p = ctypes.c_void_p()

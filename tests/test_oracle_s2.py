@@ -2,8 +2,8 @@
 
   * vision tower / decoder restatements vs the container's transformers implementation of the same Qwen2.5-VL blocks
     (seeded tiny configs, fp32, eager attention);
-  * rope_index vs the reference's own internnav/dataset/rope2d.py (when /root/reference exists) and vs the committed
-    fixture tests/golden/rope_index.json (everywhere);
+  * rope_index vs the committed fixture tests/golden/rope_index.json, the output of the reference's own
+    internnav/dataset/rope2d.py;
   * libn1b200's host-only planners (n1_rope_index, n1_vit_window_index) bit-exact vs the oracle.
 """
 import ctypes
@@ -42,18 +42,14 @@ def test_rope_index_golden():
 
 
 def test_rope_index_vs_reference():
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("reference tree not present")
-    ref = ref_loader.load_reference_rope2d()
-    for ids, grids in _cases():
+    """The oracle's full position tensor [3, 1, S] and delta against the reference's get_rope_index_25 on the same cases,
+    whose outputs tests/golden/rope_index.json records."""
+    with open(GOLD) as fh:
+        gold = json.load(fh)
+    for (ids, grids), g in zip(_cases(), gold):
         t = torch.tensor([ids])
-        g = torch.tensor(grids).reshape(-1, 3) if grids else None
-        rp, rd = ref.get_rope_index_25(2, t, g)
-        if g is None:
-            g = torch.zeros(0, 3, dtype=torch.long)
-        pos, delta = Q.rope_index(t, g)
-        assert torch.equal(rp, pos) and int(rd) == int(delta)
+        pos, delta = Q.rope_index(t, torch.tensor(grids).reshape(-1, 3) if grids else torch.zeros(0, 3, dtype=torch.long))
+        assert torch.equal(pos, torch.tensor(g["position_ids"]).unsqueeze(1)) and int(delta) == g["delta"]
 
 
 def _lib():

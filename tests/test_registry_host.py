@@ -1,6 +1,8 @@
 """Registry-level drop-in (SURVEY.md §8b) and checkpoint reading -- CPU only."""
 import json
 import os
+import subprocess
+import sys
 from types import SimpleNamespace
 
 import pytest
@@ -11,6 +13,16 @@ from internnav_b200.qwen import QWEN25VL_7B
 from oracle import agent_script
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+
+def _rerun_without_gpu(name):
+    """Runs test `name` of this file in a child pytest that sees no CUDA device, so the no-device path is also checked on a
+    machine that has one."""
+    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", "%s::%s" % (__file__, name)],
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), cwd=os.path.dirname(__file__), capture_output=True,
+                       text=True)
+    assert r.returncode == 0 and " passed" in r.stdout, r.stdout + r.stderr
+
 
 FLAT_451 = dict(  # the released config.json layout (transformers 4.51): text fields at the top level
     architectures=["InternVLAN1ForCausalLM"], model_type="internvla_n1", hidden_size=3584, num_hidden_layers=28,
@@ -58,7 +70,8 @@ def test_from_pretrained_needs_a_gpu(tmp_path):
     from safetensors.torch import save_file
     from internnav_b200.internvla_n1 import InternVLAN1ForCausalLM
     if torch.cuda.is_available():
-        pytest.skip("GPU present")
+        _rerun_without_gpu("test_from_pretrained_needs_a_gpu")
+        return
     save_file({"model.norm.weight": torch.ones(4)}, str(tmp_path / "model.safetensors"))
     (tmp_path / "config.json").write_text(json.dumps(FLAT_451))
     with pytest.raises((RuntimeError, ImportError)):
