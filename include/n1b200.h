@@ -287,6 +287,36 @@ int n1_op_patchify_depth(const void* img_f32, void* out_bf16, int n_img, int ldk
 int n1_op_adamw(void* master_f32, void* working_bf16_or_null, const void* grad_f32, void* m_f32, void* v_f32, int64_t n,
                 float lr, float beta1, float beta2, float eps, float weight_decay, int step, void* stream);
 
+/* ------------------------------------------------------------------------------------------------ training: dropout
+ * Train-mode dropout of System 1 (the reference's nn.Dropout / attention dropout_p).  A site is described by
+ * (rng, site, p): rng = device int32 [4] {seed_lo, seed_hi, step, rank}, read by the kernels at run time (a captured CUDA
+ * graph draws the masks of the step the buffer holds at replay); site = the site id of internnav_b200/dropout.py (< 2^16);
+ * p in (0, 1).  Element e of the site's tensor (row-major; attention probabilities [batch, heads, seq_q, seq_k]) is dropped
+ * iff word (e & 3) of Philox4x32-10(counter (e >> 2 low, high, site | rank << 16, step), key (seed_lo, seed_hi)) is below
+ * floor(p * 2^32); kept values are multiplied by float(1 / (1 - p)).  The backward recomputes the forward's mask.  All
+ * activations bf16. */
+/* out = residual + Z y */
+int n1_op_dropout_add(const void* residual_bf16, const void* y_bf16, void* out_bf16, int64_t n, const void* rng, int site,
+                      double p, void* stream);
+/* out = Z dy (the backward of every site; also the forward of a dropped tensor without residual) */
+int n1_op_dropout_bwd(const void* dy_bf16, void* out_bf16, int64_t n, const void* rng, int site, double p, void* stream);
+/* out[e] = 1 if element e is kept, else 0 (uint8; for tests) */
+int n1_op_dropout_mask(void* out_u8, int64_t n, const void* rng, int site, double p, void* stream);
+/* n1_op_act_fwd / n1_op_act_bwd with dropout after the activation: out = Z f(pre); out = Z dy f'(pre) */
+int n1_op_act_fwd_dropout(const void* pre_bf16, void* out_bf16, int64_t n, int act, const void* rng, int site, double p,
+                          void* stream);
+int n1_op_act_bwd_dropout(const void* pre_bf16, const void* dy_bf16, void* out_bf16, int64_t n, int act, const void* rng,
+                          int site, double p, void* stream);
+/* fixed-length multi-head attention (head_dim 48) with dropout on the probabilities: O = (softmax(S) o Z) V, and its
+ * backward (dk / dv fp32, zeroed by the caller); p == 0 runs the plain kernels */
+int n1_op_attention_dropout(const void* q, const void* k, const void* v, void* o, int ldq, int ldk, int ldv, int ldo, int heads,
+                            int head_dim, int batch, int seq_q, int seq_k, int causal, float scale, const void* rng, int site,
+                            double p, void* stream);
+int n1_op_attention_bwd_dropout(const void* q, const void* k, const void* v, const void* o, const void* dout, void* dq,
+                                void* dk_f32, void* dv_f32, int ldq, int ldk, int ldv, int ldo, int lddo, int lddq, int heads,
+                                int head_dim, int batch, int seq_q, int seq_k, int causal, float scale, const void* rng,
+                                int site, double p, void* stream);
+
 /* ------------------------------------------------------------------------------------------------ accounting
  * Kernel-launch counters are always on; with n1_prof_enable(1) every GEMM launch is additionally bracketed by CUDA
  * events on its stream (bench.py's roofline pass -- not for timed runs).  n1_prof_read synchronises, returns the sums

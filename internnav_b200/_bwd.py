@@ -4,7 +4,7 @@ Validated on the B200 against PyTorch autograd / torch.optim (tests/test_bwd_ops
 used by the training step (train_s1.py, train_step.py).  Nothing on the inference path imports this module.
 """
 import ctypes
-from ctypes import c_float, c_int, c_int64, c_void_p
+from ctypes import c_double, c_float, c_int, c_int64, c_void_p
 
 import torch
 
@@ -14,7 +14,8 @@ from ._lib import check, ptr, stream_ptr
 _bound = False
 BWD_SYMBOLS = ["n1_op_act_fwd", "n1_op_transpose", "n1_op_colsum", "n1_op_norm_bwd", "n1_op_act_bwd", "n1_op_swiglu_bwd",
                "n1_op_rope_transposed", "n1_op_attention_bwd", "n1_op_adamw", "n1_op_sgemm", "n1_op_scale_cols",
-               "n1_op_patchify_depth", "n1_op_wgrad"]
+               "n1_op_patchify_depth", "n1_op_wgrad", "n1_op_dropout_add", "n1_op_dropout_bwd", "n1_op_dropout_mask",
+               "n1_op_act_fwd_dropout", "n1_op_act_bwd_dropout", "n1_op_attention_dropout", "n1_op_attention_bwd_dropout"]
 
 
 def _L():
@@ -37,6 +38,14 @@ def _L():
         L.n1_op_patchify_depth.argtypes = [vp, vp, c_int, c_int, vp]
         L.n1_op_wgrad.argtypes = [vp, c_int, vp, c_int, c_int, c_int, c_int, vp, c_int, vp, ctypes.c_size_t, vp]
         L.n1_op_wgrad_workspace_bytes.argtypes = [c_int, c_int, c_int]
+        d = [vp, c_int, c_double, vp]                       # dropout descriptor (rng, site, p) + stream
+        L.n1_op_dropout_add.argtypes = [vp, vp, vp, c_int64] + d
+        L.n1_op_dropout_bwd.argtypes = [vp, vp, c_int64] + d
+        L.n1_op_dropout_mask.argtypes = [vp, c_int64] + d
+        L.n1_op_act_fwd_dropout.argtypes = [vp, vp, c_int64, c_int] + d
+        L.n1_op_act_bwd_dropout.argtypes = [vp, vp, vp, c_int64, c_int] + d
+        L.n1_op_attention_dropout.argtypes = [vp] * 4 + [c_int] * 10 + [c_float] + d
+        L.n1_op_attention_bwd_dropout.argtypes = [vp] * 8 + [c_int] * 12 + [c_float] + d
         L.n1_op_wgrad_workspace_bytes.restype = ctypes.c_size_t
         for n in BWD_SYMBOLS:
             getattr(L, n).restype = c_int
@@ -176,3 +185,78 @@ def patchify_depth(frames, ldk=200):
 def adamw(master, working, grad, m, v, lr, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, step=1):
     check(_L().n1_op_adamw(ptr(master), ptr(working), ptr(grad), ptr(m), ptr(v), master.numel(), lr, betas[0], betas[1], eps,
                            weight_decay, step, stream_ptr()))
+
+
+# ------------------------------------------------------------------------------------------------ dropout (training)
+# `rng`: the device int32 [4] state of internnav_b200.dropout.DropoutRNG; `site`: a site id of that module; 0 < p < 1.
+def _rng(rng):
+    assert rng.is_cuda and rng.dtype == torch.int32 and rng.numel() == 4 and rng.is_contiguous()
+    return c_void_p(rng.data_ptr())
+
+
+def _flat(t):
+    assert t.dtype == torch.bfloat16 and t.is_contiguous(), (t.dtype, t.stride())
+    return t
+
+
+def dropout_add(residual, y, rng, site, p):
+    """residual + Z y (bf16, same shape, contiguous)."""
+    assert residual.shape == y.shape
+    out = torch.empty_like(_flat(y))
+    check(_L().n1_op_dropout_add(ptr(_flat(residual)), ptr(y), ptr(out), y.numel(), _rng(rng), site, p, stream_ptr()))
+    return out
+
+
+def dropout(x, rng, site, p):
+    """Z x: a dropped tensor, and the backward of every dropout site (Z dy)."""
+    out = torch.empty_like(_flat(x))
+    check(_L().n1_op_dropout_bwd(ptr(x), ptr(out), x.numel(), _rng(rng), site, p, stream_ptr()))
+    return out
+
+
+def dropout_mask(shape, rng, site, p, device="cuda"):
+    """The keep mask of a site as uint8 [shape] (1 = kept)."""
+    out = torch.empty(shape, dtype=torch.uint8, device=device)
+    check(_L().n1_op_dropout_mask(ptr(out), out.numel(), _rng(rng), site, p, stream_ptr()))
+    return out
+
+
+def act_fwd_dropout(pre, act, rng, site, p):
+    out = torch.empty_like(_flat(pre))
+    check(_L().n1_op_act_fwd_dropout(ptr(pre), ptr(out), pre.numel(), act, _rng(rng), site, p, stream_ptr()))
+    return out
+
+
+def act_bwd_dropout(pre, dy, act, rng, site, p):
+    out = torch.empty_like(_flat(pre))
+    check(_L().n1_op_act_bwd_dropout(ptr(pre), ptr(_flat(dy)), ptr(out), pre.numel(), act, _rng(rng), site, p, stream_ptr()))
+    return out
+
+
+def attention_dropout(q, k, v, heads, head_dim, batch, seq_q, seq_k, rng, site, p, causal=False, scale=None):
+    """Fixed-length MHA (head_dim 48) with dropout on the probabilities: O = (softmax(S) o Z) V."""
+    for t in (q, k, v):
+        assert t.is_cuda and t.dtype == torch.bfloat16 and t.stride(1) == 1
+    o = torch.empty(q.shape[0], heads * head_dim, device=q.device, dtype=torch.bfloat16)
+    scale = head_dim ** -0.5 if scale is None else scale
+    vp = lambda t: c_void_p(t.data_ptr())
+    check(_L().n1_op_attention_dropout(vp(q), vp(k), vp(v), ptr(o), q.stride(0), k.stride(0), v.stride(0), o.stride(0), heads,
+                                       head_dim, batch, seq_q, seq_k, 1 if causal else 0, scale, _rng(rng), site, p,
+                                       stream_ptr()))
+    return o
+
+
+def attention_bwd_dropout(q, k, v, o, dout, heads, head_dim, batch, seq_q, seq_k, rng, site, p, causal=False, scale=None):
+    """Backward of attention_dropout (the mask recomputed): dq bf16, dk / dv fp32."""
+    dq = torch.zeros(q.shape[0], heads * head_dim, dtype=torch.bfloat16, device=q.device)
+    dk = torch.zeros(k.shape[0], heads * head_dim, dtype=torch.float32, device=q.device)
+    dv = torch.zeros_like(dk)
+    scale = head_dim ** -0.5 if scale is None else scale
+    for t in (q, k, v, o, dout):
+        assert t.is_cuda and t.dtype == torch.bfloat16 and t.stride(1) == 1
+    vp = lambda t: c_void_p(t.data_ptr())
+    check(_L().n1_op_attention_bwd_dropout(vp(q), vp(k), vp(v), vp(o), vp(dout), ptr(dq), ptr(dk), ptr(dv), q.stride(0),
+                                           k.stride(0), v.stride(0), o.stride(0), dout.stride(0), dq.stride(0), heads,
+                                           head_dim, batch, seq_q, seq_k, 1 if causal else 0, scale, _rng(rng), site, p,
+                                           stream_ptr()))
+    return dq, dk, dv

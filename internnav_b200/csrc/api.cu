@@ -485,6 +485,67 @@ int n1_op_attention_bwd(const void* q, const void* k, const void* v, const void*
     attention_bwd(p, S(stream));
   });
 }
+int n1_op_dropout_add(const void* residual, const void* y, void* out, int64_t n, const void* rng, int site, double p,
+                      void* stream) {
+  return guard([&] {
+    if (!residual || p <= 0.0) throw Error(N1_ERR_ARG, "n1_op_dropout_add: needs a residual and p > 0");
+    dropout_apply(B16(y), B16(residual), B16(out), n, make_dropout(rng, site, p), S(stream));
+  });
+}
+int n1_op_dropout_bwd(const void* dy, void* out, int64_t n, const void* rng, int site, double p, void* stream) {
+  return guard([&] {
+    if (p <= 0.0) throw Error(N1_ERR_ARG, "n1_op_dropout_bwd: p > 0");
+    dropout_apply(B16(dy), nullptr, B16(out), n, make_dropout(rng, site, p), S(stream));
+  });
+}
+int n1_op_dropout_mask(void* out_u8, int64_t n, const void* rng, int site, double p, void* stream) {
+  return guard([&] {
+    if (p <= 0.0) throw Error(N1_ERR_ARG, "n1_op_dropout_mask: p > 0");
+    dropout_mask(static_cast<uint8_t*>(out_u8), n, make_dropout(rng, site, p), S(stream));
+  });
+}
+int n1_op_act_fwd_dropout(const void* pre, void* out, int64_t n, int act, const void* rng, int site, double p, void* stream) {
+  return guard([&] {
+    if (p <= 0.0) throw Error(N1_ERR_ARG, "n1_op_act_fwd_dropout: p > 0");
+    act_fwd_dropout(B16(pre), B16(out), n, act, make_dropout(rng, site, p), S(stream));
+  });
+}
+int n1_op_act_bwd_dropout(const void* pre, const void* dy, void* out, int64_t n, int act, const void* rng, int site, double p,
+                          void* stream) {
+  return guard([&] {
+    if (p <= 0.0) throw Error(N1_ERR_ARG, "n1_op_act_bwd_dropout: p > 0");
+    act_bwd_dropout(B16(pre), B16(dy), B16(out), n, act, make_dropout(rng, site, p), S(stream));
+  });
+}
+int n1_op_attention_dropout(const void* q, const void* k, const void* v, void* o, int ldq, int ldk, int ldv, int ldo, int heads,
+                            int head_dim, int batch, int seq_q, int seq_k, int causal, float scale, const void* rng, int site,
+                            double p, void* stream) {
+  return guard([&] {
+    AttnParams a = {};
+    a.q = B16(q), a.k = B16(k), a.v = B16(v), a.o = B16(o);
+    a.ldq = ldq, a.ldk = ldk, a.ldv = ldv, a.ldo = ldo;
+    a.heads_q = a.heads_kv = heads, a.hd = head_dim, a.batch = batch, a.seq_q = seq_q, a.seq_k = seq_k;
+    a.kv_div = 1, a.causal = causal, a.scale = scale;
+    a.drop = make_dropout(rng, site, p);
+    attention(a, S(stream));
+  });
+}
+int n1_op_attention_bwd_dropout(const void* q, const void* k, const void* v, const void* o, const void* dout, void* dq,
+                                void* dk, void* dv, int ldq, int ldk, int ldv, int ldo, int lddo, int lddq, int heads,
+                                int head_dim, int batch, int seq_q, int seq_k, int causal, float scale, const void* rng,
+                                int site, double p, void* stream) {
+  return guard([&] {
+    AttnBwdParams a = {};
+    a.f.q = B16(q), a.f.k = B16(k), a.f.v = B16(v), a.f.o = const_cast<bf16*>(B16(o));
+    a.f.ldq = ldq, a.f.ldk = ldk, a.f.ldv = ldv, a.f.ldo = ldo;
+    a.f.heads_q = a.f.heads_kv = heads, a.f.hd = head_dim, a.f.batch = batch, a.f.seq_q = seq_q, a.f.seq_k = seq_k;
+    a.f.kv_div = 1, a.f.causal = causal, a.f.scale = scale;
+    a.f.drop = make_dropout(rng, site, p);
+    a.dout = B16(dout), a.lddo = lddo, a.dq = B16(dq), a.lddq = lddq;
+    a.dk = static_cast<float*>(dk), a.dv = static_cast<float*>(dv);
+    attention_bwd(a, S(stream));
+  });
+}
 int n1_traj_to_actions(const void* traj, int B, int Ns, int T, double turn_angle_rad, double step_size, int lookahead,
                        int max_actions, int cap, int32_t* ids, int32_t* count, double* mean_path, void* stream) {
   return guard([&] {

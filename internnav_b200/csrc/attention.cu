@@ -16,6 +16,9 @@
 // attention(); this file keeps the general path (any length, GQA, slotted K/V cache, head_dim 48 / 64 / 80 / 128).
 #include <stdlib.h>
 
+#include <type_traits>
+
+#include "dropout.cuh"
 #include "n1_ops.h"
 #include "n1_ptx.cuh"
 
@@ -71,8 +74,13 @@ __device__ __forceinline__ void load_tile(uint8_t* sdst, const bf16* gbase, long
   }
 }
 
-template <int HD>
-__global__ void __launch_bounds__(128) attn_kernel(const AttnParams p) {
+// DROP (training): dropout on the probabilities.  The row sum l is taken over the undropped probabilities and only the P
+// operand of O += P V is masked and scaled, so O = (softmax(S) o Z) V with Z the scaled keep mask of dropout.cuh.
+template <bool DROP>
+using AttnKParams = std::conditional_t<DROP, AttnParams, AttnCore>;
+
+template <int HD, bool DROP>
+__global__ void __launch_bounds__(128) attn_kernel(const AttnKParams<DROP> p) {
   using C = ACfg<HD>;
   extern __shared__ __align__(16) uint8_t asmem[];
   uint8_t* sQ = asmem;
@@ -119,6 +127,13 @@ __global__ void __launch_bounds__(128) attn_kernel(const AttnParams p) {
   const int lm = lane >> 3, lr = lane & 7;  // ldmatrix: matrix index / row within matrix for this lane's address
   const int row_a = q0 + warp * 16 + (lane >> 2);  // query index (within sequence) of accumulator rows c0/c1
   const int row_b = row_a + 8;                     //   and c2/c3
+  DropKey dk;
+  unsigned long long e_a = 0, e_b = 0;             // dropout element index of (row_a, key 0) / (row_b, key 0)
+  if constexpr (DROP) {
+    dk = drop_key(p.drop);
+    e_a = ((unsigned long long)(b * p.heads_q + h) * sq + row_a) * sk;
+    e_b = e_a + 8ull * sk;
+  }
 
   for (int t = 0; t < ntiles; ++t) {
     const int st = t & 1;
@@ -184,10 +199,14 @@ __global__ void __launch_bounds__(128) attn_kernel(const AttnParams p) {
     uint32_t pf[4][4];  // P as A-operand fragments: 4 k-steps of 16 keys
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
-      const float p0 = exp2f(s[i][0] - muse[0]), p1 = exp2f(s[i][1] - muse[0]);
-      const float p2 = exp2f(s[i][2] - muse[1]), p3 = exp2f(s[i][3] - muse[1]);
+      float p0 = exp2f(s[i][0] - muse[0]), p1 = exp2f(s[i][1] - muse[0]);
+      float p2 = exp2f(s[i][2] - muse[1]), p3 = exp2f(s[i][3] - muse[1]);
       ls[0] += p0 + p1;
       ls[1] += p2 + p3;
+      if constexpr (DROP) {
+        const float2 za = drop_mul2(dk, e_a + kbase + i * 8), zb = drop_mul2(dk, e_b + kbase + i * 8);
+        p0 *= za.x, p1 *= za.y, p2 *= zb.x, p3 *= zb.y;
+      }
       pf[i >> 1][(i & 1) * 2 + 0] = pack_bf16(p0, p1);
       pf[i >> 1][(i & 1) * 2 + 1] = pack_bf16(p2, p3);
     }
@@ -236,8 +255,8 @@ __global__ void __launch_bounds__(128) attn_kernel(const AttnParams p) {
 // (all heads, contiguous in memory) are staged with fully coalesced 16-byte cp.async; each warp runs QK^T, a
 // single-pass softmax and PV for its head on mma.sync; O is staged back through the Q tile and written coalesced.
 // The generic kernel above spent 4x the work on padding at these shapes (profiles/r1_ncu_small_v0_summary.txt).
-template <int NKP>  // key tiles of 16
-__global__ void __launch_bounds__(256) attn_small_kernel(const AttnParams p, const int G) {
+template <int NKP, bool DROP>  // key tiles of 16; DROP: dropout on the probabilities, as in attn_kernel
+__global__ void __launch_bounds__(256) attn_small_kernel(const AttnKParams<DROP> p, const int G) {
   constexpr int HD = 48;
   extern __shared__ __align__(16) uint8_t ssm[];
   const int heads = p.heads_q;
@@ -325,11 +344,22 @@ __global__ void __launch_bounds__(256) attn_small_kernel(const AttnParams p, con
         if (mx[r] == -INFINITY) mx[r] = 0.f;
       }
       uint32_t pf[NKP][4];
+      DropKey dk;
+      unsigned long long e_a = 0, e_b = 0;
+      if constexpr (DROP) {
+        dk = drop_key(p.drop);
+        e_a = ((unsigned long long)(b * heads + h) * sq + row_a) * sk + (lane & 3) * 2;
+        e_b = e_a + 8ull * sk;
+      }
 #pragma unroll
       for (int i = 0; i < 2 * NKP; ++i) {
-        const float p0 = exp2f(s[i][0] - mx[0]), p1 = exp2f(s[i][1] - mx[0]);
-        const float p2 = exp2f(s[i][2] - mx[1]), p3 = exp2f(s[i][3] - mx[1]);
+        float p0 = exp2f(s[i][0] - mx[0]), p1 = exp2f(s[i][1] - mx[0]);
+        float p2 = exp2f(s[i][2] - mx[1]), p3 = exp2f(s[i][3] - mx[1]);
         sum[0] += p0 + p1, sum[1] += p2 + p3;
+        if constexpr (DROP) {
+          const float2 za = drop_mul2(dk, e_a + i * 8), zb = drop_mul2(dk, e_b + i * 8);
+          p0 *= za.x, p1 *= za.y, p2 *= zb.x, p3 *= zb.y;
+        }
         pf[i >> 1][(i & 1) * 2 + 0] = pack_bf16(p0, p1);
         pf[i >> 1][(i & 1) * 2 + 1] = pack_bf16(p2, p3);
       }
@@ -371,34 +401,34 @@ __global__ void __launch_bounds__(256) attn_small_kernel(const AttnParams p, con
   }  // g
 }
 
-template <int NKP>
+template <int NKP, bool DROP = false>
 void launch_attn_small(const AttnParams& p, cudaStream_t stream) {
   const int RS = p.heads_q * 96 + 16;
   const int smem = (((p.seq_q + 15) & ~15) + 2 * NKP * 16) * RS;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaFuncSetAttribute(attn_small_kernel<NKP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (32 + 2 * NKP * 16) * (8 * 96 + 16));
+    cudaFuncSetAttribute(attn_small_kernel<NKP, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (32 + 2 * NKP * 16) * (8 * 96 + 16));
     attr_set = true;
   }
   int G = 1;  // sequences per CTA: only when they share K/V
   if (p.kv_div % 4 == 0 && p.batch % 4 == 0) G = 4;
   else if (p.kv_div % 2 == 0 && p.batch % 2 == 0) G = 2;
-  attn_small_kernel<NKP><<<p.batch / G, p.heads_q * 32, smem, stream>>>(p, G);
+  attn_small_kernel<NKP, DROP><<<p.batch / G, p.heads_q * 32, smem, stream>>>(p, G);
   prof_count_launch();
   N1_CUDA(cudaGetLastError());
 }
 
-template <int HD>
+template <int HD, bool DROP = false>
 void launch_attn(const AttnParams& p, cudaStream_t stream) {
   using C = ACfg<HD>;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaFuncSetAttribute(attn_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes);
+    cudaFuncSetAttribute(attn_kernel<HD, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::kSmemBytes);
     attr_set = true;
   }
   const int maxq = p.cu_q ? p.max_seq_q : p.seq_q;
   dim3 grid((maxq + BQ - 1) / BQ, p.heads_q, p.batch);
-  attn_kernel<HD><<<grid, 128, C::kSmemBytes, stream>>>(p);
+  attn_kernel<HD, DROP><<<grid, 128, C::kSmemBytes, stream>>>(p);
   prof_count_launch();
   N1_CUDA(cudaGetLastError());
 }
@@ -412,6 +442,20 @@ void attention(const AttnParams& p, cudaStream_t stream) {
   N1_CHECK(p.ldq % 8 == 0 && p.ldk % 8 == 0 && p.ldv % 8 == 0 && p.ldo % 2 == 0, "attention: misaligned strides");
   N1_CHECK(!p.cu_q || p.max_seq_q > 0, "attention: varlen needs max_seq_q");
   N1_CHECK(p.batch <= 65535 && p.heads_q <= 65535, "attention: grid too large");
+  if (p.drop.rng) {  // training: the NavDP decoder / Q-former attention (8 heads x 48, fixed length)
+    N1_CHECK(p.hd == 48 && !p.cu_q && !p.cu_k && !p.k_len && p.heads_q == p.heads_kv && p.kv_div == 1 && p.ldo % 8 == 0,
+             "attention: dropout needs fixed-length multi-head attention with head_dim 48, kv_div 1");
+    if (p.heads_q <= 8 && p.seq_q <= 32 && p.seq_k <= 64) {
+      const int nkp = (p.seq_k + 15) / 16;
+      if (nkp == 1) launch_attn_small<1, true>(p, stream);
+      else if (nkp == 2) launch_attn_small<2, true>(p, stream);
+      else if (nkp == 3) launch_attn_small<3, true>(p, stream);
+      else launch_attn_small<4, true>(p, stream);
+    } else {
+      launch_attn<48, true>(p, stream);
+    }
+    return;
+  }
   if (p.hd == 48 && !p.cu_q && !p.cu_k && !p.k_len && p.heads_q == p.heads_kv && p.heads_q <= 8 && p.seq_q <= 32 && p.seq_k <= 64 &&
       p.ldo % 8 == 0) {
     const int nkp = (p.seq_k + 15) / 16;

@@ -12,6 +12,12 @@
 // reductions and a deterministic result.  All products run on mma.sync.m16n8k16 (bf16 operands, fp32 accumulate) with
 // ldmatrix operand fetch: the tiles are 16 x 32 per warp, far below what a tcgen05 128-row MMA needs, and the whole
 // backward of the depth ViT is ~1.6 TFLOP per step.
+//
+// DROP (training, dropout on the probabilities; mask Z = keep / (1 - p) of dropout.cuh, recomputed from the element index):
+// the forward computed O = (P o Z) V with P = softmax(S).  Then
+//   dV = (P o Z)^T dO,   dP = (dO V^T) o Z,   dS = P o (dP - D)  with the unchanged D_i = dO_i . O_i,
+// because the softmax backward needs sum_j P_ij dP_ij = sum_j P_ij Z_ij (dO_i . V_j) = dO_i . sum_j (P o Z)_ij V_j = dO_i . O_i.
+// Phases 2 and 3 apply Z to the same (query, key) element wherever they re-form S.
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
@@ -19,6 +25,7 @@
 #include <cstdlib>
 
 #include "bwd_kernels.h"
+#include "dropout.cuh"
 #include "n1_ops.h"
 
 namespace n1 {
@@ -107,7 +114,7 @@ __device__ __forceinline__ void mm_nn32(float (&acc)[HD / 8][4], const uint32_t 
   }
 }
 
-template <int HD>
+template <int HD, bool DROP>
 __global__ void __launch_bounds__(kWarps * 32, 1) attn_bwd_mma_kernel(AttnBwdParams p, int sqp, int skp) {
   constexpr int RB = HD * 2 + 16, KS = HD / 16, NO = HD / 8;
   const AttnParams& f = p.f;
@@ -125,6 +132,12 @@ __global__ void __launch_bounds__(kWarps * 32, 1) attn_bwd_mma_kernel(AttnBwdPar
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int causal_off = sk - sq;
   const float sl2 = f.scale * 1.4426950408889634f;
+  DropKey zk;
+  unsigned long long e0 = 0;   // dropout element index of (query 0, key 0) of this (sequence, head)
+  if constexpr (DROP) {
+    zk = drop_key(f.drop);
+    e0 = (unsigned long long)(b * f.heads_q + h) * sq * sk;
+  }
 
   stage_rows<HD>(sQ, f.q + q_start * f.ldq + h * HD, f.ldq, sq, sqp);
   stage_rows<HD>(sDO, p.dout + q_start * p.lddo + h * HD, p.lddo, sq, sqp);
@@ -208,6 +221,12 @@ __global__ void __launch_bounds__(kWarps * 32, 1) attn_bwd_mma_kernel(AttnBwdPar
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
         float ds[4];
+        if constexpr (DROP) {
+          const int key0 = kc * kChunk + i * 8 + (lane & 3) * 2;
+          const float2 za = drop_mul2(zk, e0 + (unsigned long long)qa * sk + key0);
+          const float2 zb = drop_mul2(zk, e0 + (unsigned long long)qb * sk + key0);
+          dp[i][0] *= za.x, dp[i][1] *= za.y, dp[i][2] *= zb.x, dp[i][3] *= zb.y;
+        }
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
           const int key = kc * kChunk + i * 8 + (lane & 3) * 2 + (e & 1);
@@ -256,7 +275,13 @@ __global__ void __launch_bounds__(kWarps * 32, 1) attn_bwd_mma_kernel(AttnBwdPar
           const bool vis = key < sk && qi < sq && (!f.causal || key <= qi + causal_off);
           const float l = (e & 1) ? l2.y : l2.x, d = (e & 1) ? d2.y : d2.x;
           pr[e] = vis ? exp2f(st[i][e] * sl2 - l) : 0.f;
-          ds[e] = pr[e] * (dpt[i][e] - d) * f.scale;
+          if constexpr (DROP) {   // rows are keys here: the two columns of a pair are Sk elements apart
+            const float z = vis ? drop_mul(zk, e0 + (unsigned long long)qi * sk + key) : 0.f;
+            ds[e] = pr[e] * (dpt[i][e] * z - d) * f.scale;
+            pr[e] *= z;
+          } else {
+            ds[e] = pr[e] * (dpt[i][e] - d) * f.scale;
+          }
         }
         pf[i >> 1][(i & 1) * 2 + 0] = pack2(pr[0], pr[1]);
         pf[i >> 1][(i & 1) * 2 + 1] = pack2(pr[2], pr[3]);
@@ -284,14 +309,14 @@ __global__ void __launch_bounds__(kWarps * 32, 1) attn_bwd_mma_kernel(AttnBwdPar
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
-template <int HD>
+template <int HD, bool DROP = false>
 void launch(const AttnBwdParams& p, int sqp, int skp, size_t smem, cudaStream_t s) {
   static size_t attr = 0;
   if (smem > attr) {
-    N1_CUDA(cudaFuncSetAttribute(attn_bwd_mma_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    N1_CUDA(cudaFuncSetAttribute(attn_bwd_mma_kernel<HD, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr = smem;
   }
-  attn_bwd_mma_kernel<HD><<<dim3(p.f.batch, p.f.heads_q), kWarps * 32, smem, s>>>(p, sqp, skp);
+  attn_bwd_mma_kernel<HD, DROP><<<dim3(p.f.batch, p.f.heads_q), kWarps * 32, smem, s>>>(p, sqp, skp);
   prof_count_launch();
   N1_CUDA(cudaGetLastError());
 }
@@ -325,7 +350,10 @@ void attention_bwd_mma(const AttnBwdParams& p, cudaStream_t s) {
   N1_CHECK(attention_bwd_mma_supported(p), "attention_bwd_mma: unsupported problem");
   const int sqp = (p.f.seq_q + kChunk - 1) / kChunk * kChunk, skp = (p.f.seq_k + kChunk - 1) / kChunk * kChunk;
   const size_t smem = attention_bwd_mma_smem(p);
-  if (p.f.hd == 48)
+  if (p.f.drop.rng) {
+    N1_CHECK(p.f.hd == 48, "attention_bwd_mma: dropout needs head_dim 48");
+    launch<48, true>(p, sqp, skp, smem, s);
+  } else if (p.f.hd == 48)
     launch<48>(p, sqp, skp, smem, s);
   else
     launch<64>(p, sqp, skp, smem, s);

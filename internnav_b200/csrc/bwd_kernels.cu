@@ -4,6 +4,7 @@
 
 #include <math.h>
 
+#include "dropout.cuh"
 #include "n1_ptx.cuh"
 
 namespace n1 {
@@ -134,6 +135,62 @@ __global__ void act_fwd_kernel(const bf16* __restrict__ pre, bf16* __restrict__ 
   out[i] = __float2bfloat16(kind == ACT_GELU ? 0.5f * x * (1.f + erff(x * 0.70710678118654752f)) : fmaxf(x, 0.f));
 }
 
+// ---------------------------------------------------------------------------------------------- dropout (training)
+// One Philox block per thread: elements 4g .. 4g + 3 of the site's tensor (dropout.cuh).
+// out = (res ? res : 0) + Z y          (dropout_add with a residual; dropout and its backward without)
+__global__ void dropout_kernel(const bf16* __restrict__ y, const bf16* __restrict__ res, bf16* __restrict__ out, long n,
+                               const DropoutDesc d) {
+  const long g = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (4 * g >= n) return;
+  const DropKey k = drop_key(d);
+  const uint4 w = drop_words(k, (unsigned long long)g);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const long e = 4 * g + i;
+    if (e >= n) break;
+    float v = word_of(w, i) < k.thr ? 0.f : ldf(y + e) * k.scale;
+    if (res) v += ldf(res + e);
+    out[e] = __float2bfloat16(v);
+  }
+}
+
+// the keep mask as bytes (tests)
+__global__ void dropout_mask_kernel(uint8_t* __restrict__ out, long n, const DropoutDesc d) {
+  const long g = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (4 * g >= n) return;
+  const DropKey k = drop_key(d);
+  const uint4 w = drop_words(k, (unsigned long long)g);
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+    if (4 * g + i < n) out[4 * g + i] = word_of(w, i) < k.thr ? 0 : 1;
+}
+
+// activation with dropout after it (the FF inner site): forward out = Z f(pre), backward dpre = Z dy f'(pre)
+template <bool BWD>
+__global__ void act_dropout_kernel(const bf16* __restrict__ pre, const bf16* __restrict__ dy, bf16* __restrict__ out, long n,
+                                   int kind, const DropoutDesc d) {
+  const long g = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (4 * g >= n) return;
+  const DropKey k = drop_key(d);
+  const uint4 w = drop_words(k, (unsigned long long)g);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const long e = 4 * g + i;
+    if (e >= n) break;
+    const float z = word_of(w, i) < k.thr ? 0.f : k.scale;
+    const float x = ldf(pre + e);
+    float v;
+    if (BWD) {
+      const float fd = kind == ACT_GELU ? 0.5f * (1.f + erff(x * 0.70710678118654752f)) + x * 0.3989422804014327f * __expf(-0.5f * x * x)
+                                        : (x > 0.f ? 1.f : 0.f);
+      v = z * ldf(dy + e) * fd;
+    } else {
+      v = z * (kind == ACT_GELU ? 0.5f * x * (1.f + erff(x * 0.70710678118654752f)) : fmaxf(x, 0.f));
+    }
+    out[e] = __float2bfloat16(v);
+  }
+}
+
 __global__ void swiglu_bwd_kernel(const bf16* __restrict__ pre, const bf16* __restrict__ dact, bf16* __restrict__ dpre,
                                   long n) {  // n = rows * inter
   const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -227,6 +284,9 @@ constexpr int AQ = 8;  // query rows per tile
 // them ~(query heads of the group) x (query tiles) times, and the score / dP passes walk them one key per thread -- from
 // global memory those are 2-byte loads 32 rows apart (profiles/r2_launches_ddp_train_v1_summary.txt: 2.5 ms per launch in the
 // System-2 backward, 7 query heads x 304 keys x 128).
+// DROP: dropout on the probabilities (fixed-length MHA only): dV = (P o Z)^T dO, dS = P o ((dO V^T) o Z - D) with the
+// unchanged D = rowsum(dO o O) -- the identity is written out in attention_bwd_mma.cu.
+template <bool DROP>
 __global__ void __launch_bounds__(128) attn_bwd_kernel(const AttnBwdParams p, const int stage) {
   extern __shared__ float sm[];
   const AttnParams& f = p.f;
@@ -315,6 +375,12 @@ __global__ void __launch_bounds__(128) attn_bwd_kernel(const AttnBwdParams p, co
         }
         __syncthreads();
         // probabilities, dP = dO V^T, dS = P (dP - D) * scale
+        DropKey zk;
+        unsigned long long e0 = 0;   // dropout element index of (query q0, key 0)
+        if constexpr (DROP) {
+          zk = drop_key(f.drop);
+          e0 = ((unsigned long long)(b * f.heads_q + h) * sq + q0) * sk;
+        }
         for (int j = tid; j < sk; j += 128) {
           float dp[AQ];
 #pragma unroll
@@ -328,8 +394,14 @@ __global__ void __launch_bounds__(128) attn_bwd_kernel(const AttnBwdParams p, co
           for (int r = 0; r < AQ; ++r) {
             const float s = sP[r * skp + j];
             const float pr = (sL[r] > 0.f && s != -INFINITY) ? __expf(s - sM[r]) / sL[r] : 0.f;
-            sP[r * skp + j] = pr;
-            sS[r * skp + j] = pr * (dp[r] - sD[r]) * f.scale;
+            if constexpr (DROP) {
+              const float z = r < nq ? drop_mul(zk, e0 + (unsigned long long)r * sk + j) : 0.f;
+              sP[r * skp + j] = pr * z;
+              sS[r * skp + j] = pr * (dp[r] * z - sD[r]) * f.scale;
+            } else {
+              sP[r * skp + j] = pr;
+              sS[r * skp + j] = pr * (dp[r] - sD[r]) * f.scale;
+            }
           }
         }
         __syncthreads();
@@ -410,6 +482,34 @@ void act_bwd(const bf16* pre, const bf16* dy, bf16* out, long n, int kind, cudaS
   prof_count_launch();
   N1_CUDA(cudaGetLastError());
 }
+void dropout_apply(const bf16* y, const bf16* res, bf16* out, long n, const DropoutDesc& d, cudaStream_t s) {
+  N1_CHECK(d.rng && y && out && n >= 0, "dropout: bad arguments");
+  if (n == 0) return;
+  dropout_kernel<<<nblk((n + 3) / 4), 256, 0, s>>>(y, res, out, n, d);
+  prof_count_launch();
+  N1_CUDA(cudaGetLastError());
+}
+void dropout_mask(uint8_t* out, long n, const DropoutDesc& d, cudaStream_t s) {
+  N1_CHECK(d.rng && out && n >= 0, "dropout_mask: bad arguments");
+  if (n == 0) return;
+  dropout_mask_kernel<<<nblk((n + 3) / 4), 256, 0, s>>>(out, n, d);
+  prof_count_launch();
+  N1_CUDA(cudaGetLastError());
+}
+void act_fwd_dropout(const bf16* pre, bf16* out, long n, int kind, const DropoutDesc& d, cudaStream_t s) {
+  N1_CHECK(kind == ACT_GELU || kind == ACT_RELU, "act_fwd: GELU or ReLU");
+  N1_CHECK(d.rng, "act_fwd_dropout: no RNG state");
+  act_dropout_kernel<false><<<nblk((n + 3) / 4), 256, 0, s>>>(pre, nullptr, out, n, kind, d);
+  prof_count_launch();
+  N1_CUDA(cudaGetLastError());
+}
+void act_bwd_dropout(const bf16* pre, const bf16* dy, bf16* out, long n, int kind, const DropoutDesc& d, cudaStream_t s) {
+  N1_CHECK(kind == ACT_GELU || kind == ACT_RELU, "act_bwd: GELU or ReLU");
+  N1_CHECK(d.rng, "act_bwd_dropout: no RNG state");
+  act_dropout_kernel<true><<<nblk((n + 3) / 4), 256, 0, s>>>(pre, dy, out, n, kind, d);
+  prof_count_launch();
+  N1_CUDA(cudaGetLastError());
+}
 void swiglu_bwd(const bf16* pre, const bf16* dact, bf16* dpre, long rows, int inter, cudaStream_t s) {
   swiglu_bwd_kernel<<<nblk(rows * inter), 256, 0, s>>>(pre, dact, dpre, rows * inter);
   prof_count_launch();
@@ -464,13 +564,26 @@ void attention_bwd(const AttnBwdParams& p, cudaStream_t s) {
                        (reinterpret_cast<uintptr_t>(f.v) & 3) == 0;
   const int stage = aligned && smem + kv_bytes <= 200 * 1024 ? 1 : 0;
   if (stage) smem += kv_bytes;
+  dim3 grid(f.batch / f.kv_div, f.heads_kv);
+  if (f.drop.rng) {
+    N1_CHECK(!f.cu_q && !f.cu_k && !f.k_len && f.kv_div == 1 && f.heads_q == f.heads_kv,
+             "attention_bwd: dropout needs fixed-length multi-head attention, kv_div 1");
+    static size_t attr_d = 0;
+    if (smem > attr_d) {
+      N1_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      attr_d = smem;
+    }
+    attn_bwd_kernel<true><<<grid, 128, smem, s>>>(p, stage);
+    prof_count_launch();
+    N1_CUDA(cudaGetLastError());
+    return;
+  }
   static size_t attr = 0;
   if (smem > attr) {
-    N1_CUDA(cudaFuncSetAttribute(attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    N1_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr = smem;
   }
-  dim3 grid(f.batch / f.kv_div, f.heads_kv);
-  attn_bwd_kernel<<<grid, 128, smem, s>>>(p, stage);
+  attn_bwd_kernel<false><<<grid, 128, smem, s>>>(p, stage);
   prof_count_launch();
   N1_CUDA(cudaGetLastError());
 }

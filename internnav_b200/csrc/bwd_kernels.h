@@ -30,6 +30,14 @@ void norm_bwd(const bf16* dy, int ld_dy, const bf16* x, int ld_x, const float* w
 void act_fwd(const bf16* pre, bf16* out, long n, int kind, cudaStream_t s);
 // Elementwise activation backward on the saved pre-activation: out = dy * f'(pre); kind: ACT_GELU (exact erf) / ACT_RELU
 void act_bwd(const bf16* pre, const bf16* dy, bf16* out, long n, int kind, cudaStream_t s);
+// Dropout of the training step (mask contract: dropout.cuh; d.rng must be set):
+//   dropout_apply   out = (res ? res : 0) + Z y   -- a residual branch with dropout, a dropped tensor, or the backward Z dy
+//   dropout_mask    out[e] = keep(e) as 0 / 1 bytes (tests)
+//   act_*_dropout   the FF inner site: out = Z f(pre) ; dpre = Z dy f'(pre)  (the pre-activation stays the only saved tensor)
+void dropout_apply(const bf16* y, const bf16* res, bf16* out, long n, const DropoutDesc& d, cudaStream_t s);
+void dropout_mask(uint8_t* out, long n, const DropoutDesc& d, cudaStream_t s);
+void act_fwd_dropout(const bf16* pre, bf16* out, long n, int kind, const DropoutDesc& d, cudaStream_t s);
+void act_bwd_dropout(const bf16* pre, const bf16* dy, bf16* out, long n, int kind, const DropoutDesc& d, cudaStream_t s);
 // SwiGLU backward: pre [R, 2I] interleaved (gate_j, up_j) pre-activations, dact [R, I] -> dpre [R, 2I] interleaved
 void swiglu_bwd(const bf16* pre, const bf16* dact, bf16* dpre, long rows, int inter, cudaStream_t s);
 // out[r, c] = x[r, c] * gamma[c] (+ add[r, c])   -- layer scale and its backward share this
@@ -47,6 +55,7 @@ void sgemm_small(const float* A, int lda, int trans_a, const float* B, int ldb, 
 // element (row, head, d) at ptr[row * ld + head * hd + d]; fixed or var-len / slotted sequences; GQA; bottom-right
 // causal.  Outputs: dq bf16 (same addressing as q with lddq), dk / dv fp32 [rows_k, heads_kv * hd] dense, ZEROED by the
 // caller when several launches accumulate into them (kv_div > 1: query sequences sharing one K/V sequence).
+// f.drop set: the backward of attention with dropout on the probabilities (fixed-length MHA, head_dim 48 on the tensor cores).
 struct AttnBwdParams {
   AttnParams f;          // forward description; f.o is the forward output
   const bf16* dout;      // gradient of f.o, same layout (lddo)

@@ -77,8 +77,30 @@ int prof_read_shapes(int* mnk, long* count, double* ms, int cap);
 void layernorm(const bf16* x, int ldx, bf16* y, int ldy, const float* w, const float* b, int rows, int D,
                float eps, int rms, cudaStream_t stream);
 
+// ------------------------------------------------------------------------------------------- dropout
+// One dropout site of the training step (mask contract: dropout.cuh).  rng == nullptr: no dropout.
+struct DropoutDesc {
+  const uint32_t* rng = nullptr;  // device {seed_lo, seed_hi, step, rank}
+  float p = 0.f;
+  uint32_t thr = 0;               // floor(p * 2^32)
+  float scale = 1.f;              // float(1 / (1 - p))
+  int site = 0;                   // site id (internnav_b200/dropout.py), < 2^16
+};
+inline DropoutDesc make_dropout(const void* rng, int site, double p) {
+  if (!(p >= 0.0 && p < 1.0) || site < 0 || site >= 65536) throw Error(-2, "dropout: p must be in [0, 1), site in [0, 2^16)");
+  DropoutDesc d;
+  if (p == 0.0) return d;
+  if (!rng) throw Error(-2, "dropout: p > 0 needs the device RNG state");
+  d.rng = static_cast<const uint32_t*>(rng), d.p = (float)p, d.site = site;
+  d.thr = (uint32_t)(p * 4294967296.0);
+  d.scale = (float)(1.0 / (1.0 - p));
+  return d;
+}
+
 // ------------------------------------------------------------------------------------------- attention
-struct AttnParams {
+// The sequence description the forward kernels without dropout take by value (kept apart from the dropout fields so that
+// their parameter block, and with it their code, stays as it was).
+struct AttnCore {
   const bf16* q;  // element (row, head, d) at q[row * ldq + head * hd + d]
   const bf16* k;
   const bf16* v;
@@ -97,6 +119,9 @@ struct AttnParams {
   int k_slot;            //   [kb * k_slot, kb * k_slot + k_len[kb]); overrides cu_k / seq_k
   long total_rows;       // optional: rows of the packed q / k / v buffers (var-len self-attention); > 0 lets head_dim 128
                          //   sequences of <= 320 tokens take the tcgen05 kernel (attention_tc.cu), which needs it for TMA
+};
+struct AttnParams : AttnCore {
+  DropoutDesc drop;      // dropout on the probabilities (training): fixed-length MHA with head_dim 48 only; off by default
 };
 void attention(const AttnParams& p, cudaStream_t stream);
 // tcgen05 / TMEM / TMA attention for head_dim 128, var-len self-attention with <= 320 keys per sequence (attention_tc.cu)

@@ -15,11 +15,19 @@ the library / a B200).  tests/test_train_s1_host.py drives this same schedule wi
 the `ops` contract on the CPU and checks every gradient against the oracle -- that validates the schedule, not the
 kernels.  The kernels are validated on the B200 by tests/test_bwd_ops_gpu.py (op level, System-2 half, and the whole step
 against the oracle chain; profiles/r2_bwd_ops_parity.log).
+
+Train-mode dropout (`S1TrainStep(..., dropout=p)`, p > 0): at every site of internnav_b200/dropout.py the schedule calls the
+dropout primitives of the backend with `drop = (DropoutRNG, site id, p)` -- `dropout_add` at the residual branches,
+`dropout` on the cond / action embeddings and on the gradients flowing back through a site, `act_fwd` / `act_bwd` and
+`attention` / `attention_bwd` with a `drop` argument.  With p == 0 the schedule issues exactly the calls it issues without.
 """
 import math
 
 import torch
 import torch.nn.functional as F
+
+from .dropout import (ACTION, COND, CROSS_PROBS, DROPOUT1, DROPOUT2, DROPOUT3, FF_INNER, SELF_PROBS, DropoutRNG, decoder_site,
+                      qformer_site)
 
 ACT_GELU, ACT_RELU = 1, 2
 
@@ -57,17 +65,35 @@ class GpuOps:
     def norm_bwd(self, dy, x, w, eps):
         return self._bwd.norm_bwd(dy, x, w, eps)
 
-    def attention(self, q, k, v, heads, hd, batch, sq, sk, causal):
+    def attention(self, q, k, v, heads, hd, batch, sq, sk, causal, drop=None):
+        if drop is not None:
+            rng, site, p = drop
+            return self._bwd.attention_dropout(q, k, v, heads, hd, batch, sq, sk, rng.dev, site, p, causal=causal)
         return self._lib.attention(q, k, v, heads, heads, hd, batch, sq, sk, causal=causal)
 
-    def attention_bwd(self, q, k, v, o, do, heads, hd, batch, sq, sk, causal):
+    def attention_bwd(self, q, k, v, o, do, heads, hd, batch, sq, sk, causal, drop=None):
+        if drop is not None:
+            rng, site, p = drop
+            return self._bwd.attention_bwd_dropout(q, k, v, o, do, heads, hd, batch, sq, sk, rng.dev, site, p, causal=causal)
         return self._bwd.attention_bwd(q, k, v, o, do, heads, heads, hd, batch, sq, sk, causal=causal)
 
-    def act_fwd(self, pre, kind):
+    def act_fwd(self, pre, kind, drop=None):
+        if drop is not None:
+            return self._bwd.act_fwd_dropout(pre, kind, drop[0].dev, drop[1], drop[2])
         return self._bwd.act_fwd(pre, kind)
 
-    def act_bwd(self, pre, dy, kind):
+    def act_bwd(self, pre, dy, kind, drop=None):
+        if drop is not None:
+            return self._bwd.act_bwd_dropout(pre, dy, kind, drop[0].dev, drop[1], drop[2])
         return self._bwd.act_bwd(pre, dy, kind)
+
+    def dropout(self, x, drop):
+        """Z x: a dropped tensor, or the gradient flowing back through a dropout site."""
+        return self._bwd.dropout(x, drop[0].dev, drop[1], drop[2])
+
+    def dropout_add(self, residual, y, drop):
+        """residual + Z y: a residual branch with dropout."""
+        return self._bwd.dropout_add(residual, y, drop[0].dev, drop[1], drop[2])
 
     def wgrad(self, dy, x):
         """dy [M, N]^T @ x [M, K] -> fp32 [N, K]: in place on MN-major operand tiles when the rows are aligned
@@ -98,12 +124,18 @@ def _pad8(x):
 class S1TrainStep:
     """params: {reference tensor name: fp32 tensor} (the state_dict keys of NavDP_Policy_DPT_CriticSum_DAT)."""
 
-    def __init__(self, params, ops, heads=8, layers=16, frames=2, K=20):
+    def __init__(self, params, ops, heads=8, layers=16, frames=2, K=20, dropout=0.0, rng=None):
+        """dropout: the reference's train-mode p (0.1) at every site of internnav_b200/dropout.py; rng: its DropoutRNG (the
+        masks of micro-batch rng.step), by default seed 0 on the parameters' device."""
         self.ops, self.heads, self.layers, self.frames, self.K = ops, heads, layers, frames, K
         self.p32 = dict(params)
         self._alias_in_proj()
         self.w = {}           # working copies in the kernel dtype (refresh() after every optimizer step)
         self.refresh()
+        self.dropout = float(dropout)
+        if not 0.0 <= self.dropout < 1.0:
+            raise ValueError("dropout must be in [0, 1)")
+        self.rng = rng if rng is not None or self.dropout == 0 else DropoutRNG(0, device=self.w["layernorm.weight"].device)
         self._resample = {}
         self._touched = set()   # tensors that received a gradient in the current step (torch.optim skips the others)
 
@@ -120,6 +152,32 @@ class S1TrainStep:
                 self.w[k] = self.ops.cast(v)
 
     # ---- primitives on the backend ----------------------------------------------------------------------------
+    def _drop(self, site):
+        """The dropout descriptor of a site, or None when the step runs without dropout."""
+        return (self.rng, site, self.dropout) if self.dropout > 0 else None
+
+    def _residual(self, x, y, site):
+        """x + dropout(y) in the kernel dtype."""
+        d = self._drop(site)
+        if d is None:
+            return self.ops.cast(x.float() + y.float())
+        return self.ops.dropout_add(x.contiguous(), y.contiguous(), d)
+
+    def _drop_grad(self, dy, site):
+        """The gradient through a dropout site (dy itself without dropout)."""
+        d = self._drop(site)
+        return dy if d is None else self.ops.dropout(dy.contiguous(), d)
+
+    def _act(self, pre, kind, site):
+        d = self._drop(site)
+        x = pre.reshape(-1, pre.shape[-1])
+        return (self.ops.act_fwd(x, kind) if d is None else self.ops.act_fwd(x, kind, drop=d)).reshape(pre.shape)
+
+    def _act_bwd(self, pre, dy, kind, site):
+        d = self._drop(site)
+        x, g = pre.reshape(-1, pre.shape[-1]).contiguous(), dy.reshape(-1, pre.shape[-1]).contiguous()
+        return self.ops.act_bwd(x, g, kind) if d is None else self.ops.act_bwd(x, g, kind, drop=d)
+
     def _f32(self, name):
         return self.p32[name].to(self.w[name].device, torch.float32)
 
@@ -168,7 +226,7 @@ class S1TrainStep:
         self._acc(g, name + ".bias", db)
         return dx.reshape(shp)
 
-    def mha(self, name, q_in, kv_in, causal=False):
+    def mha(self, name, q_in, kv_in, causal=False, site=None):
         """nn.MultiheadAttention with packed in_proj; q_in [B, Sq, D], kv_in [B, Sk, D] (kv_in is q_in for self-attention)."""
         D = q_in.shape[-1]
         B, Sq, Sk = q_in.shape[0], q_in.shape[1], kv_in.shape[1]
@@ -179,16 +237,23 @@ class S1TrainStep:
             q = self.lin(name + ".in_proj", q_in, rows=slice(0, D)).reshape(B * Sq, D)
             kv = self.lin(name + ".in_proj", kv_in, rows=slice(D, 3 * D)).reshape(B * Sk, 2 * D)
             k, v = kv[:, :D], kv[:, D:]
-        o = self.ops.attention(q, k, v, self.heads, D // self.heads, B, Sq, Sk, causal)
+        d = None if site is None else self._drop(site)
+        if d is None:
+            o = self.ops.attention(q, k, v, self.heads, D // self.heads, B, Sq, Sk, causal)
+        else:
+            o = self.ops.attention(q, k, v, self.heads, D // self.heads, B, Sq, Sk, causal, drop=d)
         y = self.lin(name + ".out_proj", o.reshape(B, Sq, D))
-        return y, (q_in, kv_in, q, k, v, o, causal)
+        return y, (q_in, kv_in, q, k, v, o, causal, d)
 
     def mha_bwd(self, name, saved, dy, g):
-        q_in, kv_in, q, k, v, o, causal = saved
+        q_in, kv_in, q, k, v, o, causal, d = saved
         D = q_in.shape[-1]
         B, Sq, Sk = q_in.shape[0], q_in.shape[1], kv_in.shape[1]
         do = self.lin_bwd(name + ".out_proj", o.reshape(B, Sq, D), dy, g).reshape(B * Sq, D).contiguous()
-        dq, dk, dv = self.ops.attention_bwd(q, k, v, o, do, self.heads, D // self.heads, B, Sq, Sk, causal)
+        if d is None:
+            dq, dk, dv = self.ops.attention_bwd(q, k, v, o, do, self.heads, D // self.heads, B, Sq, Sk, causal)
+        else:
+            dq, dk, dv = self.ops.attention_bwd(q, k, v, o, do, self.heads, D // self.heads, B, Sq, Sk, causal, drop=d)
         dk, dv = dk.to(dq.dtype), dv.to(dq.dtype)
         if kv_in is q_in:
             dqkv = torch.cat((dq, dk, dv), dim=1).reshape(B, Sq, 3 * D)
@@ -287,31 +352,33 @@ class S1TrainStep:
         self._acc(g, p + "patch_embed.proj.bias", ops.colsum(dpatch))
 
     # ---- Q-former layer (post-norm, ReLU; navdp_backbone.py L148) ---------------------------------------------
-    def post_layer(self, p, x, mem):
-        a1, m1 = self.mha(p + "self_attn", x, x)
-        s1 = self.ops.cast(x.float() + a1.float())
+    def post_layer(self, p, x, mem, layer=0):
+        site = lambda off: qformer_site(layer, off)                                       # noqa: E731
+        a1, m1 = self.mha(p + "self_attn", x, x, site=site(SELF_PROBS))
+        s1 = self._residual(x, a1, site(DROPOUT1))
         x1 = self.ln(p + "norm1", s1, 1e-5)
-        a2, m2 = self.mha(p + "multihead_attn", x1, mem)
-        s2 = self.ops.cast(x1.float() + a2.float())
+        a2, m2 = self.mha(p + "multihead_attn", x1, mem, site=site(CROSS_PROBS))
+        s2 = self._residual(x1, a2, site(DROPOUT2))
         x2 = self.ln(p + "norm2", s2, 1e-5)
         f1 = self.lin(p + "linear1", x2)
-        act = self.ops.act_fwd(f1.reshape(-1, f1.shape[-1]), ACT_RELU).reshape(f1.shape)
+        act = self._act(f1, ACT_RELU, site(FF_INNER))
         f2 = self.lin(p + "linear2", act)
-        s3 = self.ops.cast(x2.float() + f2.float())
-        return self.ln(p + "norm3", s3, 1e-5), (m1, s1, m2, s2, x2, f1, act, s3)
+        s3 = self._residual(x2, f2, site(DROPOUT3))
+        return self.ln(p + "norm3", s3, 1e-5), (m1, s1, m2, s2, x2, f1, act, s3, layer)
 
     def post_layer_bwd(self, p, saved, dy, g):
         ops = self.ops
-        m1, s1, m2, s2, x2, f1, act, s3 = saved
+        m1, s1, m2, s2, x2, f1, act, s3, layer = saved
+        site = lambda off: qformer_site(layer, off)                                       # noqa: E731
         d = self.ln_bwd(p + "norm3", s3, dy, g, 1e-5)
-        dact = self.lin_bwd(p + "linear2", act, d, g)
-        df1 = ops.act_bwd(f1.reshape(-1, f1.shape[-1]).contiguous(), dact.reshape(-1, f1.shape[-1]).contiguous(), ACT_RELU)
+        dact = self.lin_bwd(p + "linear2", act, self._drop_grad(d, site(DROPOUT3)), g)
+        df1 = self._act_bwd(f1, dact, ACT_RELU, site(FF_INNER))
         dx2 = ops.cast(d.float() + self.lin_bwd(p + "linear1", x2, df1.reshape(f1.shape), g).float())
         d = self.ln_bwd(p + "norm2", s2, dx2, g, 1e-5)
-        dq, dmem = self.mha_bwd(p + "multihead_attn", m2, d, g)
+        dq, dmem = self.mha_bwd(p + "multihead_attn", m2, self._drop_grad(d, site(DROPOUT2)), g)
         dx1 = ops.cast(d.float() + dq.float())
         d = self.ln_bwd(p + "norm1", s1, dx1, g, 1e-5)
-        dq, _ = self.mha_bwd(p + "self_attn", m1, d, g)
+        dq, _ = self.mha_bwd(p + "self_attn", m1, self._drop_grad(d, site(DROPOUT1)), g)
         return ops.cast(d.float() + dq.float()), dmem
 
     # ---- model pieces ------------------------------------------------------------------------------------------
@@ -328,7 +395,7 @@ class S1TrainStep:
         x = ops.cast(self._f32(p + "former_query.weight")[: self.frames * 16].unsqueeze(0).expand(B, -1, -1))
         tape = []
         for i in range(2):
-            x, s = self.post_layer("%sformer_net.layers.%d." % (p, i), x, token)
+            x, s = self.post_layer("%sformer_net.layers.%d." % (p, i), x, token, layer=i)
             tape.append(s)
         return self.lin(p + "project_layer", x), (vsave, tape, x, B, T)
 
@@ -398,21 +465,24 @@ class S1TrainStep:
         cond = torch.cat([time_emb, goal.float(), rgbd.float()], dim=1) + self._f32("cond_pos_embed")[:, :M]
         cond = ops.cast(cond.repeat_interleave(Ns, dim=0))
         x = ops.cast(x + self._f32("out_pos_embed")[:, :T])
+        if self.dropout > 0:        # NavDP.drop on the condition and action embeddings (navdp.py L305-307)
+            cond, x = ops.dropout(cond, self._drop(COND)), ops.dropout(x, self._drop(ACTION))
         tape = []
         for i in range(self.layers):
             p = "decoder.layers.%d." % i
+            site = lambda off: decoder_site(i, off)                                        # noqa: E731
             h1 = self.ln(p + "norm1", x, 1e-5)
-            a1, m1 = self.mha(p + "self_attn", h1, h1, causal=True)
-            x1 = ops.cast(x.float() + a1.float())
+            a1, m1 = self.mha(p + "self_attn", h1, h1, causal=True, site=site(SELF_PROBS))
+            x1 = self._residual(x, a1, site(DROPOUT1))
             h2 = self.ln(p + "norm2", x1, 1e-5)
-            a2, m2 = self.mha(p + "multihead_attn", h2, cond)
-            x2 = ops.cast(x1.float() + a2.float())
+            a2, m2 = self.mha(p + "multihead_attn", h2, cond, site=site(CROSS_PROBS))
+            x2 = self._residual(x1, a2, site(DROPOUT2))
             h3 = self.ln(p + "norm3", x2, 1e-5)
             f1 = self.lin(p + "linear1", h3)
-            act = ops.act_fwd(f1.reshape(-1, f1.shape[-1]), ACT_GELU).reshape(f1.shape)
+            act = self._act(f1, ACT_GELU, site(FF_INNER))
             f2 = self.lin(p + "linear2", act)
             tape.append((x, m1, x1, m2, x2, h3, f1, act))
-            x = ops.cast(x2.float() + f2.float())
+            x = self._residual(x2, f2, site(DROPOUT3))
         hN = self.ln("layernorm", x, 1e-5)
         y = ops.sgemm(hN.float().reshape(-1, hN.shape[-1]), self._f32("action_head.weight"), trans_b=True).reshape(R, T, 3) \
             + self._f32("action_head.bias")                                                      # D -> 3
@@ -429,15 +499,19 @@ class S1TrainStep:
         for i in reversed(range(self.layers)):
             p = "decoder.layers.%d." % i
             x, m1, x1, m2, x2, h3, f1, act = tape[i]
-            dact = self.lin_bwd(p + "linear2", act, dx, g)
-            df1 = ops.act_bwd(f1.reshape(-1, f1.shape[-1]).contiguous(), dact.reshape(-1, f1.shape[-1]).contiguous(), ACT_GELU)
+            site = lambda off: decoder_site(i, off)                                        # noqa: E731
+            dact = self.lin_bwd(p + "linear2", act, self._drop_grad(dx, site(DROPOUT3)), g)
+            df1 = self._act_bwd(f1, dact, ACT_GELU, site(FF_INNER))
             dh3 = self.lin_bwd(p + "linear1", h3, df1.reshape(f1.shape), g)
             dx = ops.cast(dx.float() + self.ln_bwd(p + "norm3", x2, dh3, g, 1e-5).float())
-            dq, dkv = self.mha_bwd(p + "multihead_attn", m2, dx, g)
+            dq, dkv = self.mha_bwd(p + "multihead_attn", m2, self._drop_grad(dx, site(DROPOUT2)), g)
             dcond = dcond + dkv.float()
             dx = ops.cast(dx.float() + self.ln_bwd(p + "norm2", x1, dq, g, 1e-5).float())
-            dq, _ = self.mha_bwd(p + "self_attn", m1, dx, g)
+            dq, _ = self.mha_bwd(p + "self_attn", m1, self._drop_grad(dx, site(DROPOUT1)), g)
             dx = ops.cast(dx.float() + self.ln_bwd(p + "norm1", x, dq, g, 1e-5).float())
+        if self.dropout > 0:
+            dx = ops.dropout(dx.contiguous(), self._drop(ACTION))
+            dcond = ops.dropout(ops.cast(dcond), self._drop(COND)).float()
         dxf = dx.float()
         gop = torch.zeros_like(self.p32["out_pos_embed"], dtype=torch.float32, device=dxf.device)
         gop[:, :T] = dxf.sum(0, keepdim=True)

@@ -16,10 +16,15 @@ exchange happens on the last micro-batch only, like DDP's no_sync), global-norm 
 (`max_grad_norm=1`, train_dual_system.sh), an LR-schedule hook (`lr_schedule(step) -> lr`; `warmup_cosine` below is the
 Trainer's `cosine` with `warmup_ratio`), AdamW with decoupled decay, parameters without gradient untouched.
 
-DEVIATION (stated, not hidden): dropout.  The reference trains in train() mode, so p=0.1 dropout is active on the cond /
-action embeddings (navdp.py L305-307), in the 16 decoder layers and in the 2 Q-former layers.  This step runs WITHOUT
-dropout (the kernels have no mask inputs); oracle and goldens are eval-mode.  It is therefore the reference's
-optimisation step with dropout p=0.  There is no CPU path.
+Dropout: the reference trains in train() mode, so p = 0.1 dropout is active on the cond / action embeddings (navdp.py
+L305-307), in the 16 decoder layers and in the 2 Q-former layers (attention probabilities, the three residual branches, the
+FF inner activation).  `DualSystemTrainer(..., dropout=0.1)` reproduces that: every site of internnav_b200/dropout.py runs
+the dropout kernels, with masks drawn from Philox4x32-10 keyed by `dropout_seed` and counted by (site, data-parallel rank,
+micro-batch step) -- the contract of csrc/dropout.cuh, restated in oracle/philox.py.  The masks cannot equal torch's RNG
+stream; the parity tests inject the same masks into the oracle and into the reference module
+(tests/golden/s1_training_dropout_reference.npz).  `dropout=0` (the default) is the reference's step with dropout off, and
+issues exactly the kernels of a trainer without dropout.  The goal compressor (dropout 0.0), both DINOv2 ViTs and the frozen
+System-2 decoder have no dropout.  There is no CPU path.
 """
 import math
 from collections import OrderedDict
@@ -28,6 +33,7 @@ import torch
 
 from . import _bwd, _lib
 from .ddp import GradientBuckets
+from .dropout import DropoutRNG
 from .train_s1 import GpuOps, S1TrainStep
 
 
@@ -46,9 +52,11 @@ def warmup_cosine(base_lr, total_steps, warmup_ratio=0.03, min_ratio=0.0):
 class DualSystemTrainer:
     def __init__(self, model, navdp_state_dict, latent_queries, lr=1e-4, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0,
                  bucket_cap_mb=100, process_group=None, max_grad_norm=None, lr_schedule=None, accumulation_steps=1,
-                 graph_s1=False):
+                 graph_s1=False, dropout=0.0, dropout_seed=0):
         """model: internnav_b200.internvla_n1.InternVLAN1ForCausalLM with weights loaded (the frozen parts are used from
-        it); navdp_state_dict: {reference name: tensor} for `model.navdp.*`; latent_queries [1, n_query, H]."""
+        it); navdp_state_dict: {reference name: tensor} for `model.navdp.*`; latent_queries [1, n_query, H].
+        dropout: System 1's train-mode dropout p (0.1 reproduces the reference's training; 0 turns it off); dropout_seed:
+        the key of the mask stream (each micro-batch and each data-parallel rank draws its own masks)."""
         self.model = model
         dev = model.device
         if dev.type != "cuda":
@@ -59,7 +67,11 @@ class DualSystemTrainer:
             if v.is_floating_point():
                 self.masters[k] = v.detach().to(dev, torch.float32).clone()
         self.latent = latent_queries.detach().to(dev, torch.float32).clone()
-        self.s1 = S1TrainStep(self.masters, GpuOps(str(dev)))
+        dist_on = torch.distributed.is_available() and torch.distributed.is_initialized()
+        rank = torch.distributed.get_rank(process_group) if dist_on else 0
+        self.dropout_rng = DropoutRNG(dropout_seed, rank, dev) if dropout > 0 else None
+        self._dropout_step = 0          # micro-batches run so far: the `step` word of the mask counter
+        self.s1 = S1TrainStep(self.masters, GpuOps(str(dev)), dropout=dropout, rng=self.dropout_rng)
         trainable = OrderedDict((k, (tuple(v.shape), torch.float32)) for k, v in self.masters.items()
                                 if not k.startswith("rgbd_encoder.rgb_model."))
         trainable["model.latent_queries"] = (tuple(self.latent.shape), torch.float32)
@@ -147,9 +159,15 @@ class DualSystemTrainer:
         _lib.lib().n1_prof_add(nodes["gemm_launches"], nodes["total_launches"])
         return loss, touched, dhs
 
-    def loss_and_grads(self, batch, noise, timesteps):
+    def _set_dropout_step(self, step):
+        if self.dropout_rng is not None:
+            self.dropout_rng.set_step(step)
+
+    def loss_and_grads(self, batch, noise, timesteps, dropout_step=None):
         """Parity entry point: (loss, {name: fp32 gradient}, TRAJ states) for one batch; no exchange, no update.
-        batch: the collated dict of internnav_b200.training.collate_traj_batch (tensors may live on the host)."""
+        batch: the collated dict of internnav_b200.training.collate_traj_batch (tensors may live on the host).
+        dropout_step: the micro-batch whose dropout masks are used (default: the next one); the counter does not advance."""
+        self._set_dropout_step(self._dropout_step if dropout_step is None else dropout_step)
         hs = self._s2_forward(batch)
         loss, grads, dhs = self._s1_forward_backward(batch, hs, noise, timesteps)
         grads["model.latent_queries"] = self.model._s2.train_backward(dhs).reshape(self.latent.shape)
@@ -172,6 +190,8 @@ class DualSystemTrainer:
         hs = self._s2_forward(batch)
         if pe:
             pe[1].record()
+        self._set_dropout_step(self._dropout_step)      # a static input of the graphed step, copied before its replay
+        self._dropout_step += 1
         if self.graph_s1:
             loss, grads, dhs = self._s1_graphed(batch, hs, noise, timesteps)
         else:
@@ -245,6 +265,21 @@ class DualSystemTrainer:
         ev[3].synchronize()
         return {"overlapped_launch_ms": ev[0].elapsed_time(ev[1]), "exposed_ms": ev[2].elapsed_time(ev[3]),
                 "s2_backward_window_ms": ev[1].elapsed_time(ev[2])}
+
+    # ------------------------------------------------------------------ dropout mask stream
+    def dropout_state(self):
+        """What a resumed run needs to continue the dropout mask stream (save it beside the optimizer state, as HF Trainer
+        saves its RNG states): {"p", "seed", "step"}; `step` counts the micro-batches run."""
+        rng = self.dropout_rng
+        return {"p": self.s1.dropout, "seed": rng.seed if rng is not None else None, "step": self._dropout_step}
+
+    def load_dropout_state(self, state):
+        """Continue the mask stream of `dropout_state()` (this process keeps its own data-parallel rank)."""
+        if float(state["p"]) != self.s1.dropout:
+            raise ValueError("dropout p of the saved state (%r) differs from this trainer's (%r)" % (state["p"], self.s1.dropout))
+        if self.dropout_rng is not None:
+            self.dropout_rng.seed = int(state["seed"])
+        self._dropout_step = int(state["step"])
 
     # ------------------------------------------------------------------ export
     def state_dict(self):
